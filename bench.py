@@ -2,7 +2,17 @@
 """bench.py -- the UAPS unlabeled-batch hot path on B200, one JSON line (contract: task brief (4)).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config neu|dagm|kosdd2]
-                    [--no-train-step] [--no-sweep] [--no-other-configs]
+                    [--no-train-step] [--no-sweep] [--no-other-configs] [--dump-outputs DIR]
+
+--steps K sets the timed steps of the headline blocks only: the headline loss and the headline configuration's training
+iteration.  The other configurations, the sweep, the inference block and the host-logits footnote keep their own fixed
+counts (the footnote takes K clamped to 3..10).
+
+--dump-outputs DIR writes, after the timed steps, what the headline loss path returned in its last step as
+DIR/<name>.npy (see DUMP_SAMPLE).  Its inputs depend only on the arguments and its outputs are bitwise reproducible, so
+two builds can be compared output for output.
+The training iteration is not dumped: it sums its BatchNorm statistics with atomics, whose order varies, so it differs run
+to run in the last bits, and the iterations amplify that.
 
 Headline workload (BASELINE.json configs[1] at the shape of configs[2]'s unlabeled batch): the fused
 pseudo-label + KL-uncertainty + weighted CE/Dice loss, forward + backward, K=4 decoders, C=4
@@ -61,6 +71,33 @@ CONFIGS = {
 CW1 = CW2 = 0.1
 CPU_TRAIN_B = 4                        # bounded CPU sample of the full iteration: 4 + 4 images
 FT = (16, 32, 64, 128, 256)
+DUMP_SAMPLE = 1 << 22                  # --dump-outputs keeps this many elements of a larger output (16 MB of float32)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_sample(ts):
+    """The tensors `ts` flattened and concatenated as a host array, or, when that is longer than DUMP_SAMPLE, the
+    DUMP_SAMPLE elements at a fixed set of positions (drawn with seed 0, in increasing order)."""
+    total = sum(t.numel() for t in ts)
+    if total <= DUMP_SAMPLE:
+        return torch.cat([t.detach().reshape(-1) for t in ts]).cpu().numpy()
+    idx = np.sort(np.random.default_rng(0).choice(total, DUMP_SAMPLE, replace=False))
+    out, start = [], 0
+    for t in ts:
+        sel = idx[(idx >= start) & (idx < start + t.numel())] - start
+        out.append(t.detach().reshape(-1)[torch.from_numpy(sel).to(t.device)].cpu())
+        start += t.numel()
+    return torch.cat(out).numpy()
+
+
+def write_dump(path, arrays):
+    """arrays: {name: float32 / float64 array} -> path/<name>.npy."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values()), {k: a.dtype for k, a in arrays.items()}
+    nbytes = sum(a.nbytes for a in arrays.values())
+    assert nbytes <= DUMP_MAX_BYTES, nbytes
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def workload_name(c):
@@ -279,8 +316,9 @@ def run_reference(args):
 
 
 # ---- GPU arm ---------------------------------------------------------------------------------------------------
-def loss_bench(c, dev, lib, L, group, world, rank, xchg, steps, warmup, seed_off=0):
-    """Device-resident fused loss fwd+bwd through the C ABI: (ms_total, t_pass1, t_pass2, n_events)."""
+def loss_bench(c, dev, lib, L, group, world, rank, xchg, steps, warmup, seed_off=0, dump=None):
+    """Device-resident fused loss fwd+bwd through the C ABI: (ms_total, t_pass1, t_pass2, n_events).  `dump` (a dict)
+    receives the last step's scalars, partial sums and a sample of the logits' gradient."""
     import torch.distributed as dist
     K, C, B, H, W = c["K"], c["C"], c["B"], c["H"], c["W"]
     N = B * H * W
@@ -341,6 +379,8 @@ def loss_bench(c, dev, lib, L, group, world, rank, xchg, steps, warmup, seed_off
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total, t1, t2 = t.tolist()
+    if dump is not None:
+        dump.update(loss_scalars=sc.cpu().numpy(), loss_sums=sums.cpu().numpy(), loss_grad_logits=dump_sample(dz))
     del z, dz
     return ms_total, t1, t2, len(evs), EV_EVERY
 
@@ -474,7 +514,7 @@ def train_step_bench(c, dev, group, world, rank, steps: int = 8, warmup: int = 4
     flop = 3.0 * model_flops_per_image(cin, C, K, H, W) * 2 * batch            # fprop + dgrad + wgrad, labeled + unlabeled
     tfs = flop / (ms * 1e-3) / 1e12
     mode = ("captured CUDA graph" if trainer._graphs else "device-state eager") if trainer.state is not None else "host scalars, eager launches"
-    out = {"iters_per_s": 1e3 / ms, "ms_per_iter": ms, "images_per_s": 2 * batch * world * 1e3 / ms,
+    out = {"iters_per_s": 1e3 / ms, "ms_per_iter": ms, "steps": steps, "images_per_s": 2 * batch * world * 1e3 / ms,
            "unlabeled_pixels_per_s": batch * H * W * world * 1e3 / ms, "unit": "iters/s", "loss": float(loss_h),
            "h2d_bytes_per_iter": xl_h.numel() * 4 * 2 + yl_h.numel() * 8, "d2h_bytes_per_iter": 4,
            "tflop_per_iter_per_gpu": flop / 1e12,
@@ -620,8 +660,11 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
+    dump = {} if args.dump_outputs and rank == 0 else None
     # ---- headline: device-resident fused loss ------------------------------------------------------------------
-    ms_total, t1, t2, n_ev, ev_every = loss_bench(c, dev, lib, L, group, world, rank, xchg, args.steps, warmup)
+    ms_total, t1, t2, n_ev, ev_every = loss_bench(c, dev, lib, L, group, world, rank, xchg, args.steps, warmup, dump=dump)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     roof, kernels, value, ms_step = loss_roofline(c, ms_total, t1, t2, args.steps, world, peak, peak_src)
     footnote = e2e_host_logits(c, dev, group, world, mix_w, max(3, min(args.steps, 10)))
 
@@ -636,7 +679,7 @@ def run_ours(args):
     train, others = None, {}
     if not args.no_train_step:
         try:
-            train = train_step_bench(c, dev, group, world, rank)
+            train = train_step_bench(c, dev, group, world, rank, steps=args.steps)
         except Exception as e:                                  # noqa: BLE001
             train = {"error": repr(e)[:300]}
         if not args.no_other_configs:
@@ -736,14 +779,20 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline blocks (the loss and the training iteration "
+                                                          "of --config); the other blocks keep fixed counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="neu", choices=sorted(CONFIGS))
     ap.add_argument("--no-train-step", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline loss path's outputs of its last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's GPU path; --impl reference has none")
     if args.impl == "reference":
         run_reference(args)
     else:
