@@ -191,6 +191,28 @@ int uaps_loss_pass2(const float* const* z, int K, int B, int C, int64_t HW,
                     float* const* dz, int flags, const float* wcw_dev /* nullable, as in pass 1 */, cudaStream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Ensemble inference head: the test-time uncertainty of the K decoders (UAPS-Testing.ipynb cell 11) from the
+ * expressions of the uncertainty loss, per pixel, with no loss sums:
+ *   labels[b,hw]            = argmax_c q (uint8, lowest index on ties), q = (((p_0 + p_1) + ...) / K) and
+ *                             p_k = softmax(z_k) (UAPS_train.py:186-189, 223) -- bit-exact with torch.argmax(q, 1)
+ *                             by the same near-tie rule as the pseudo-label of pass 1;
+ *   uncertainty[b,hw]       = (1/K) sum_k V_k, V_k = sum_c KLDiv(log_softmax(z_k), q) (:226-236), the per-pixel
+ *                             term of the uncertainty loss (:241-243);
+ *   image_uncertainty[b]    = mean of uncertainty over the HW pixels of image b, summed in fp64 in a fixed order
+ *                             (bitwise reproducible);
+ *   mean_prob[b,c,hw]       = q.
+ * z: host array of K device pointers [B,C,HW] fp32 (1 <= K <= UAPS_KMAX, 2 <= C <= UAPS_CMAX, any HW).
+ * uncertainty, image_uncertainty and mean_prob are nullable.  image_uncertainty needs a workspace of at least
+ * uaps_ensemble_workspace_bytes(K, C, B, HW) bytes, 8-byte aligned; every launch writes the part it reads, so it
+ * needs no initialisation and the call can be captured into a CUDA graph and replayed.
+ * Algorithmic HBM bytes per pixel: 4KC read + 1 (label) + 4 (uncertainty) written, + 4C with mean_prob.
+ * ------------------------------------------------------------------------------------------- */
+size_t uaps_ensemble_workspace_bytes(int K, int C, int B, int64_t HW);
+int uaps_ensemble_head(const float* const* z, int K, int B, int C, int64_t HW, uint8_t* labels, float* uncertainty,
+                       float* image_uncertainty, float* mean_prob, void* workspace, size_t workspace_bytes,
+                       cudaStream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Encoder-feature perturbations (utilities/UAPS_unet.py:156-185, applied at :227-231).
  * x, y: [B, C, HW] fp32 (C*HW = `chw` elements per sample where only that matters).
  * Randomness is either INJECTED (a caller-provided tensor, used for parity with the reference's

@@ -60,6 +60,8 @@ _SIGNATURES = {
     "uaps_xchg_status": (_i, [_vp, _vp, _vp]),
     "uaps_loss_finalize": (_i, [_vp, _i, _i, _i64, _f, _f, _i, _vp, _vp]),
     "uaps_loss_pass2": (_i, [_vp, _i, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "uaps_ensemble_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i64]),
+    "uaps_ensemble_head": (_i, [_vp, _i, _i, _i, _i64, _vp, _vp, _vp, _vp, _vp, C.c_size_t, _vp]),
     "uaps_feature_noise": (_i, [_vp, _vp, _u64, _f, _vp, _i, _i64, _vp]),
     "uaps_dropout": (_i, [_vp, _vp, _u64, _d, _vp, _i64, _vp]),
     "uaps_fdrop_stats": (_i, [_vp, _i, _i, _i64, _vp, _vp, _vp]),

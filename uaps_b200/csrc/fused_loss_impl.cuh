@@ -170,6 +170,11 @@ __device__ __forceinline__ void log2_softmax_underflow_fix(const float (&z)[C], 
         if (t[c] < kLg2Floor) l2[c] = t[c] - l2s;      // lg2(p) is exact enough above the floor; below it p may have flushed
 }
 
+// torch's `acc / K` for the mean prediction (UAPS_train.py:223): ATen divides a CUDA tensor by a python scalar as a
+// multiplication by the fp32-rounded reciprocal (div_true_kernel_cuda), so this is also what kl_terms computes
+template <int K>
+__device__ __forceinline__ float mean_of_sum(float acc) { return __fmul_rn(acc, 1.0f / K); }
+
 // torch-order argmax of the Dirichlet mix (UAPS_train.py:251-255), every rounding reproduced
 template <int K, int C>
 __device__ __forceinline__ int argmax_exact(const float (&p)[K][C], const float (&w)[K]) {
@@ -187,18 +192,42 @@ __device__ __forceinline__ int argmax_exact(const float (&p)[K][C], const float 
 }
 
 // Near-tie slow path: re-reads the pixel's logits (L1/L2 hits) so the hot loop keeps nothing alive for it.
-template <int K, int C>
-__device__ __noinline__ int argmax_exact_gmem(const LossArgs& a, size_t pix_off) {
-    float p[K][C], w[K];
+// MEAN: the argmax of the mean prediction q = (((p_0 + p_1) + p_2) + ...) / K (:223) instead of the mix, in the same
+// torch order (the sum runs along the decoders, so only C partial sums stay live).  Args: LossArgs, or any argument
+// block with the same z[] / HW fields (and w_dev / w unless MEAN).
+template <int K, int C, bool MEAN = false, typename Args>
+__device__ __noinline__ int argmax_exact_gmem(const Args& a, size_t pix_off) {
+    if constexpr (MEAN) {
+        float acc[C];
 #pragma unroll
-    for (int k = 0; k < K; ++k) {
-        float z[C], l[C];
+        for (int k = 0; k < K; ++k) {
+            float z[C], p[C], l[C];
 #pragma unroll
-        for (int c = 0; c < C; ++c) z[c] = __ldg(a.z[k] + pix_off + (size_t)c * a.HW);
-        softmax_exact<C>(z, p[k], l);
-        w[k] = a.w_dev != nullptr ? a.w_dev[k] : a.w[k];
+            for (int c = 0; c < C; ++c) z[c] = __ldg(a.z[k] + pix_off + (size_t)c * a.HW);
+            softmax_exact<C>(z, p, l);
+#pragma unroll
+            for (int c = 0; c < C; ++c) acc[c] = k == 0 ? p[c] : __fadd_rn(acc[c], p[c]);
+        }
+        int y = 0;
+        float best = mean_of_sum<K>(acc[0]);
+#pragma unroll
+        for (int c = 1; c < C; ++c) {
+            const float q = mean_of_sum<K>(acc[c]);
+            if (q > best) { best = q; y = c; }
+        }
+        return y;
+    } else {
+        float p[K][C], w[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            float z[C], l[C];
+#pragma unroll
+            for (int c = 0; c < C; ++c) z[c] = __ldg(a.z[k] + pix_off + (size_t)c * a.HW);
+            softmax_exact<C>(z, p[k], l);
+            w[k] = a.w_dev != nullptr ? a.w_dev[k] : a.w[k];
+        }
+        return argmax_exact<K, C>(p, w);
     }
-    return argmax_exact<K, C>(p, w);
 }
 
 // mean prediction (UAPS_train.py:223) and KL maps (:226-236): V_k = sum_c xlogy(q,q) - q * l_kc, E_k = exp(-V_k).
@@ -289,9 +318,40 @@ __device__ __forceinline__ void pixel_forward(const float (&z)[K][C], const floa
     }
 }
 
+// Inference form of pixel_forward (default arithmetic): softmaxes, mean prediction and KL maps as above, but the label
+// is the argmax of the mean prediction q itself (UAPS_train.py:223 followed by argmax), bit-exact with torch's
+// argmax(q, 1) by the same near-tie rule.  st.E is left to dead-code elimination.
+template <int K, int C, typename Args>
+__device__ __forceinline__ void pixel_mean_forward(const float (&z)[K][C], const Args& a, size_t pix_off, PixelState<K, C>& st) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) softmax_fast<C, false>(z[k], st.p[k], st.l[k]);
+    kl_terms<K, C, false, false>(st);
+    int y = 0;
+    float best = st.q[0], second = -1.f;
+#pragma unroll
+    for (int c = 1; c < C; ++c) {
+        if (st.q[c] > best) { second = best; best = st.q[c]; y = c; }
+        else second = fmaxf(second, st.q[c]);
+    }
+    float vs = st.V[0];
+#pragma unroll
+    for (int k = 1; k < K; ++k) vs += st.V[k];
+    const bool tie = !(best - second > kTieMargin);
+    const bool bad = !(fabsf(vs) < 1e30f);
+    if (__builtin_expect(tie || bad, 0)) {
+        if (tie) y = argmax_exact_gmem<K, C, true>(a, pix_off);
+        if (bad) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) log2_softmax_underflow_fix<C>(z[k], st.l[k]);
+            kl_terms<K, C, false, true>(st);
+        }
+    }
+    st.y = y;
+}
+
 // K*C independent vector loads of one pixel group (one per class plane of every decoder)
-template <int K, int C, int VEC>
-__device__ __forceinline__ void load_group(const LossArgs& a, unsigned g, float (&zv)[K][C][VEC]) {
+template <int K, int C, int VEC, typename Args>
+__device__ __forceinline__ void load_group(const Args& a, unsigned g, float (&zv)[K][C][VEC]) {
     const unsigned b = g / a.groups_per_image;
     const unsigned hw = (g - b * a.groups_per_image) * VEC;
     const size_t base = (size_t)b * C * a.HW + hw;

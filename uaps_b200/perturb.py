@@ -276,15 +276,21 @@ class _Perturb3NhwcFn(torch.autograd.Function):
 
 
 def perturb3_nhwc(x: torch.Tensor, *, u: Optional[float] = None, seed: Optional[int] = None,
-                  uniform_range: float = 0.3, p: float = 0.5, outputs=(True, True, True), aliases: int = 0):
+                  uniform_range: float = 0.3, p: float = 0.5, outputs=(True, True, True), aliases: int = 0,
+                  seed_dev: Optional[int] = None, u_dev: Optional[int] = None):
     """Channels-last bf16 ``perturb3``: (FeatureNoise, Dropout, FeatureDropout) of one feature map in one pass.
     ``outputs``: which of the three copies to produce (None for the others) -- a 4th / 5th auxiliary decoder (the K = 5
     ablation) calls it again for ONE more copy of the perturbation family it re-uses, with a fresh draw.
     ``aliases``: that many extra outputs that are x itself -- hand them to the UNPERTURBED consumers of x (main decoder, next
     level's max-pool) and the backward kernel sums their gradients too, instead of autograd's separate accumulation passes.
     Inside a device-resident iteration (``stepctx.current().state``) the Philox key and the threshold u come from the
-    device step state; otherwise they are drawn from ``uaps_b200.perturb.generator`` on the host."""
+    device step state; otherwise they are drawn from ``uaps_b200.perturb.generator`` on the host.
+    ``seed_dev`` / ``u_dev``: device addresses of a uint64 Philox key and an fp32 threshold read by the kernel at run time
+    (the key is added to ``seed``, default 0; u is replaced), so a captured graph can be replayed with fresh draws."""
     from . import stepctx
+    if seed_dev is not None or u_dev is not None:
+        return _Perturb3NhwcFn.apply(x, int(seed or 0), float(uniform_range), float(p), float(np.float32(u or 0.8)),
+                                     seed_dev, u_dev, tuple(bool(o) for o in outputs), int(aliases))
     sc = stepctx.current()
     seed_dev = u_dev = None
     if sc is not None and sc.state is not None and seed is None and u is None:

@@ -20,6 +20,7 @@ from __future__ import annotations
 
 from typing import Dict, List, Optional, Sequence
 
+import numpy as np
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -34,6 +35,11 @@ ENC_DROPOUT = (0.05, 0.1, 0.2, 0.3, 0.5)    # :214
 _AUX_KINDS = ("noise", "dropout", "fdrop")  # :227, :229, :231; a 4th/5th aux decoder re-uses them in order
 BN_NREP = 8                                 # replicas of the BatchNorm sums a conv epilogue accumulates into (spreads the atomics)
 BN_FUSE_MAX_COUT = int(__import__("os").environ.get("UAPS_BN_FUSE_MAX_COUT", "32"))   # widest layer whose conv epilogue takes the statistics
+
+
+def _check_hw(x: torch.Tensor) -> None:
+    if x.shape[-1] % 16 or x.shape[-2] % 16:
+        raise RuntimeError("H and W must be multiples of 16 (four 2x poolings; the reference fails in torch.cat)")
 
 
 def _holder(**children: nn.Module) -> nn.Module:
@@ -230,27 +236,58 @@ class UNet_UAPS(nn.Module):
         b = (conv.bias.detach().float() - bn.running_mean.detach().float()) * s + bn.bias.detach().float()
         return w.contiguous(), b.contiguous()
 
+    def _block_plan(self, blk, cin_split=None):
+        cc = blk.conv_conv
+        w0, b0 = self._fold_bn(cc.get_submodule("0"), cc.get_submodule("1"))
+        w4, b4 = self._fold_bn(cc.get_submodule("4"), cc.get_submodule("5"))
+        return PackedConv(w0, b0, cin_split=cin_split), PackedConv(w4, b4)
+
+    def _decoder_plan(self, dm: nn.Module):
+        dec = []
+        for i in range(1, 5):
+            up = dm.get_submodule(f"up{i}")
+            c2 = FT_CHNS[4 - i]
+            dec.append((PackedConv(up.conv1x1.weight, up.conv1x1.bias), *self._block_plan(up.conv, cin_split=c2)))
+        return dec, PackedConv(dm.out_conv.weight, dm.out_conv.bias)
+
     def _inference_plan(self):
-        """Packed, BN-folded layers of encoder + main decoder (built lazily, dropped by train() / load_state_dict())."""
+        """Packed, BN-folded layers of encoder + main decoder (built lazily, dropped by train() / load_state_dict()), and
+        a dict that receives the auxiliary decoders' layers when an ensemble first needs them (``_aux_plan``)."""
         plan = getattr(self, "_infer_plan", None)
         if plan is not None:
             return plan
-        def block(blk, cin_split=None):
-            cc = blk.conv_conv
-            w0, b0 = self._fold_bn(cc.get_submodule("0"), cc.get_submodule("1"))
-            w4, b4 = self._fold_bn(cc.get_submodule("4"), cc.get_submodule("5"))
-            return PackedConv(w0, b0, cin_split=cin_split), PackedConv(w4, b4)
-        enc = [block(self.encoder.in_conv)] + \
-              [block(self.encoder.get_submodule(f"down{lvl}").maxpool_conv.get_submodule("1")) for lvl in range(1, 5)]
-        dec = []
-        md = self.main_decoder
-        for i in range(1, 5):
-            up = md.get_submodule(f"up{i}")
-            c2 = FT_CHNS[4 - i]
-            dec.append((PackedConv(up.conv1x1.weight, up.conv1x1.bias), *block(up.conv, cin_split=c2)))
-        out = PackedConv(md.out_conv.weight, md.out_conv.bias)
-        self._infer_plan = (enc, dec, out)
+        enc = [self._block_plan(self.encoder.in_conv)] + \
+              [self._block_plan(self.encoder.get_submodule(f"down{lvl}").maxpool_conv.get_submodule("1")) for lvl in range(1, 5)]
+        dec, out = self._decoder_plan(self.main_decoder)
+        self._infer_plan = (enc, dec, out, {})
         return self._infer_plan
+
+    def _aux_plan(self, a: int):
+        aux = self._inference_plan()[3]
+        if a not in aux:
+            aux[a] = self._decoder_plan(self.get_submodule(f"aux_decoder{a}"))
+        return aux[a]
+
+    @staticmethod
+    def _encode_folded(x, enc):
+        """Folded encoder: five levels of channels-last bf16 feature maps [B,H_l,W_l,C_l]."""
+        cur = to_nhwc_bf16(x)                                                # [B,H,W,16]
+        feats = []
+        for lvl, (c0, c4) in enumerate(enc):
+            if lvl:
+                cur = maxpool2(cur.permute(0, 3, 1, 2)).permute(0, 2, 3, 1)
+            cur = c4(c0(cur, slope=0.01), slope=0.01)
+            feats.append(cur)
+        return feats
+
+    @staticmethod
+    def _decode_folded(feats, dec, out):
+        """Folded decoder over channels-last feature maps: fp32 NCHW logits."""
+        cur = feats[4]
+        for i, (c1x1, c0, c4) in enumerate(dec, start=1):
+            up = upsample2x(c1x1(cur).permute(0, 3, 1, 2)).permute(0, 2, 3, 1)
+            cur = c4(c0(feats[4 - i], up, slope=0.01), slope=0.01)
+        return out(cur, out_nchw_f32=True)
 
     def train(self, mode: bool = True):
         self._infer_plan = None                       # weights are about to change: drop the folded copies
@@ -272,19 +309,8 @@ class UNet_UAPS(nn.Module):
         4 upsamples -- no BatchNorm or activation pass touches HBM.  In training mode (batch statistics) and on the
         fp32 path it falls back to the ordinary layers."""
         if self.compute == "bf16" and not self.training:
-            enc, dec, out = self._inference_plan()
-            cur = to_nhwc_bf16(x)                                            # [B,H,W,16]
-            feats = []
-            for lvl, (c0, c4) in enumerate(enc):
-                if lvl:
-                    cur = maxpool2(cur.permute(0, 3, 1, 2)).permute(0, 2, 3, 1)
-                cur = c4(c0(cur, slope=0.01), slope=0.01)
-                feats.append(cur)
-            cur = feats[4]
-            for i, (c1x1, c0, c4) in enumerate(dec, start=1):
-                up = upsample2x(c1x1(cur).permute(0, 3, 1, 2)).permute(0, 2, 3, 1)
-                cur = c4(c0(feats[4 - i], up, slope=0.01), slope=0.01)
-            return out(cur, out_nchw_f32=True)
+            enc, dec, out, _ = self._inference_plan()
+            return self._decode_folded(self._encode_folded(x, enc), dec, out)
         if self.compute == "bf16":
             return self._decode16(self._encode16(x, None), self.main_decoder)
         return self.decode(self.encode(x), self.main_decoder)
@@ -319,6 +345,121 @@ class UNet_UAPS(nn.Module):
         graph.replay()
         return static_out
 
+    # ---- ensemble inference: every decoder, label map + uncertainty maps (DESIGN.md f5) -------------------------------
+    def _ensemble_calls(self) -> int:
+        """Perturbation launches of an ensemble forward: one per level for auxiliary decoders 1-3 together, then one per
+        level for each of decoders 4 and 5."""
+        return 5 * (1 + max(0, self.n_aux - 3))
+
+    def _ensemble_draws(self, seed: Optional[int]) -> np.ndarray:
+        """Host int64 [2, n]: row 0 the Philox keys, row 1 the FeatureDropout thresholds (fp32 in the low 4 bytes), one
+        column per perturbation launch (see ``predict_uncertainty`` for the order)."""
+        if seed is None:
+            P._mix_rank_once()
+            rng = P.generator
+        else:
+            rng = np.random.default_rng(int(seed))
+        n = self._ensemble_calls()
+        draws = np.zeros((2, n), dtype=np.int64)
+        u32 = draws[1].view(np.float32)                       # little-endian: float i sits at index 2i
+        for i in range(n):
+            draws[0, i] = rng.integers(0, 2 ** 63 - 1)
+            u32[2 * i] = rng.uniform(0.7, 0.9)
+        return draws
+
+    def _ensemble_logits16(self, x: torch.Tensor, draws: torch.Tensor) -> List[torch.Tensor]:
+        """Folded encoder once; main decoder on the clean features, auxiliary decoder a on its perturbed copy of them
+        (the reference's eval-mode forward, UAPS_unet.py:224-233); the draws are read from the device tensor ``draws``."""
+        enc, dec, out, _ = self._inference_plan()
+        feats = self._encode_folded(x, enc)
+        keys, uth = draws[0], draws[1]
+
+        def perturb(i, f, outputs):
+            return P.perturb3_nhwc(f.permute(0, 3, 1, 2), outputs=outputs, seed_dev=keys[i].data_ptr(),
+                                   u_dev=uth[i].data_ptr())
+
+        live = tuple(a <= self.n_aux for a in (1, 2, 3))
+        per_level = [perturb(lvl, f, live) for lvl, f in enumerate(feats)]
+        logits = [self._decode_folded(feats, dec, out)]
+        for a in range(1, self.n_aux + 1):
+            kind = _AUX_KINDS[(a - 1) % 3]
+            if a <= 3:
+                pf = [t[a - 1] for t in per_level]
+            else:                                             # a fresh draw of the family, as _forward16 does
+                sel = tuple(k == kind for k in _AUX_KINDS)
+                pf = [perturb(5 * (a - 3) + lvl, f, sel)[_AUX_KINDS.index(kind)] for lvl, f in enumerate(feats)]
+            logits.append(self._decode_folded([t.permute(0, 2, 3, 1) for t in pf], *self._aux_plan(a)))
+        return logits
+
+    def _check_ensemble_input(self, x: torch.Tensor) -> None:
+        if self.n_aux == 0:
+            raise ValueError("predict_uncertainty needs at least one auxiliary decoder (n_aux >= 1)")
+        _check_hw(x)
+
+    @torch.no_grad()
+    def predict_uncertainty(self, x: torch.Tensor, *, seed: Optional[int] = None, return_probs: bool = False):
+        """Ensemble inference (UAPS-Testing.ipynb cell 11; DESIGN.md f5): every decoder's logits, then
+        ``ensemble.ensemble_uncertainty`` -- ``(labels uint8 [B,H,W], uncertainty fp32 [B,H,W], image_uncertainty fp32 [B],
+        mean_prob fp32 [B,C,H,W] | None)``: the argmax of the decoders' mean softmax, the mean KL divergence of each
+        decoder from that mean per pixel (0 where they agree) and its per-image mean.
+
+        As in the reference's eval-mode forward, the main decoder sees the clean encoder features and auxiliary decoder a
+        a perturbed copy (FeatureNoise, Dropout(0.5), FeatureDropout for a = 1, 2, 3; a = 4, 5 a fresh draw of the first
+        two families); the encoder's own dropout is off.
+
+        bf16 path in eval mode: the folded encoder runs once, every decoder through BN-folded packed convs, the
+        perturbations are the Philox kernels of training, and the head is one ``uaps_ensemble_head`` launch.  The random
+        draws are n = 5 * (1 + max(0, n_aux - 3)) (Philox key, FeatureDropout u) pairs, one per perturbation launch, in
+        the order: levels 0-4 of the shared launch for decoders 1-3, then levels 0-4 for decoder 4, then for decoder 5.
+        Launch i takes key_i = rng.integers(0, 2**63 - 1), then u_i = rng.uniform(0.7, 0.9) (rounded to fp32), where rng
+        is ``numpy.random.default_rng(seed)`` for an int ``seed`` and ``uaps_b200.perturb.generator`` for ``seed=None``.
+        In training mode and on the fp32 path it runs ``forward(x)`` (whose draws come from the generator; ``seed`` is
+        not used there) and the same head."""
+        self._check_ensemble_input(x)
+        from .ensemble import ensemble_uncertainty
+        if self.compute == "bf16" and not self.training:
+            draws = torch.from_numpy(self._ensemble_draws(seed)).to(x.device)       # one host-to-device copy
+            logits = self._ensemble_logits16(x, draws)
+        else:
+            logits = self.forward(x)
+        return ensemble_uncertainty(logits, return_probs=return_probs)
+
+    @torch.no_grad()
+    def predict_uncertainty_graphed(self, x: torch.Tensor, *, seed: Optional[int] = None):
+        """``predict_uncertainty`` replayed from a CUDA graph (bf16 path, eval mode), one graph per input shape, as
+        ``predict_graphed``.  The draws live in a static device buffer that receives fresh draws (from ``seed`` as
+        ``predict_uncertainty`` derives them) before every replay.  The returned tensors are the graph's static output
+        buffers: the next call with the same shape overwrites them."""
+        if self.compute != "bf16" or self.training:
+            return self.predict_uncertainty(x, seed=seed)
+        self._check_ensemble_input(x)
+        from .ensemble import ensemble_uncertainty
+        key = ("uncertainty", tuple(x.shape), x.device.index)
+        cache = self.__dict__.setdefault("_graphs", {})
+        entry = cache.get(key)
+        host_draws = torch.from_numpy(self._ensemble_draws(seed))
+        if entry is None or entry[4] is not self._inference_plan():
+            static_in = torch.empty_like(x, dtype=torch.float32)
+            static_in.copy_(x)
+            static_draws = host_draws.to(x.device)
+            run = lambda: ensemble_uncertainty(self._ensemble_logits16(static_in, static_draws))
+            side = torch.cuda.Stream(device=x.device)
+            side.wait_stream(torch.cuda.current_stream(x.device))
+            with torch.cuda.stream(side):                       # warm-up off the capture: lazy inits, plans, allocator
+                for _ in range(2):
+                    run()
+            torch.cuda.current_stream(x.device).wait_stream(side)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                static_out = run()
+            entry = (graph, static_in, static_draws, static_out, self._inference_plan())
+            cache[key] = entry
+        graph, static_in, static_draws, static_out, _ = entry
+        static_in.copy_(x)
+        static_draws.copy_(host_draws)
+        graph.replay()
+        return static_out
+
     def decoders(self) -> List[nn.Module]:
         return [self.main_decoder] + [self.get_submodule(f"aux_decoder{a}") for a in range(1, self.n_aux + 1)]
 
@@ -326,8 +467,7 @@ class UNet_UAPS(nn.Module):
     def forward(self, x: torch.Tensor, rand: Optional[Dict[str, list]] = None):
         """UNet_UAPS.forward (:224-233).  ``rand`` optionally injects every random draw:
         {"enc_keep": 5 masks, "noise": 5 tensors [C_l,H_l,W_l], "aux2_keep": 5 masks, "u": 5 floats}."""
-        if x.shape[-1] % 16 or x.shape[-2] % 16:
-            raise RuntimeError("H and W must be multiples of 16 (four 2x poolings; the reference fails in torch.cat)")
+        _check_hw(x)
         if self.compute == "bf16":
             return self._forward16(x, rand)
         feats = self.encode(x, None if rand is None else rand["enc_keep"])
