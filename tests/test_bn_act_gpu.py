@@ -38,6 +38,7 @@ def test_bn_lrelu_matches_torch(B, C, H, W):
 
 
 def test_fused_dropout_is_consistent_between_forward_and_backward():
+    from oracle.philox_ref import bn_keep, keep_scale
     from uaps_b200.bn_act import bn_lrelu_dropout
     dev = torch.device("cuda:0")
     C = 32
@@ -53,6 +54,14 @@ def test_fused_dropout_is_consistent_between_forward_and_backward():
         assert torch.allclose(out.float()[kept], (base.float() * scale)[kept], rtol=2e-2, atol=1e-3)
         # same seed -> same mask
         assert torch.equal(bn_lrelu_dropout(y, bn, p, seed=7) != 0, kept)
-        # gradient flows only through kept elements' contribution: d(sum out)/dy is finite and non-zero
+        # the mask is Philox(seed 7, stream 21) of the chunk index, bit for bit (oracle/philox_ref.py)
+        want = torch.from_numpy(bn_keep(7, y.numel() // C, C, p)).to(dev)
+        rows = lambda t: t.permute(0, 2, 3, 1).reshape(-1, C)
+        nz = rows(base) != 0
+        assert torch.equal(rows(kept)[nz], want[nz])
+        # backward regenerates it: d beta = sum(g * keep * keep_scale * leaky_relu'(z)) over the oracle's mask
+        bn.weight.grad = bn.bias.grad = None
         out.float().sum().backward()
-        assert torch.isfinite(yo.grad.float()).all() and yo.grad.float().abs().sum().item() > 0
+        assert torch.isfinite(yo.grad.float()).all()
+        d = torch.where(rows(base) > 0, 1.0, 0.01).double() * want.double() * float(keep_scale(p))
+        assert torch.allclose(bn.bias.grad.double(), d.sum(0), rtol=1e-5, atol=1e-3)

@@ -144,6 +144,15 @@ struct BnParams {
 };
 __device__ __forceinline__ uint64_t eff_seed(const BnParams& p) { return p.seed + (p.seed_dev != nullptr ? *p.seed_dev : 0ull); }
 
+// z = y * sc + sh with sc = gamma * rstd, sh = beta - mean * sc, from the SAVED fp32 mean / rstd and rounded the same way in
+// the forward and both backward kernels: an element whose z lies within an ulp of 0 then takes one LeakyReLU branch in
+// all three (three differently rounded shifts disagreed in about a third of the channels, so such an element could be
+// differentiated on the other branch than the one the forward took).
+__device__ __forceinline__ void bn_scale_shift(float gamma, float beta, float mean, float rstd, float& sc, float& sh) {
+    sc = __fmul_rn(gamma, rstd);
+    sh = __fmaf_rn(-mean, sc, beta);
+}
+
 // forward: a = dropout(leaky_relu(gamma * (y - mean) * rstd + beta))
 __global__ void __launch_bounds__(BT) bn_act_kernel(const uint4* __restrict__ y, uint4* __restrict__ out, const BnParams p) {
     __shared__ float s_scale[256], s_shift[256];
@@ -158,8 +167,7 @@ __global__ void __launch_bounds__(BT) bn_act_kernel(const uint4* __restrict__ y,
         double var = s2 / n - mean * mean;
         if (var < 0.0) var = 0.0;
         const float rstd = (float)(1.0 / sqrt(var + (double)p.eps));
-        s_scale[c] = p.gamma[c] * rstd;
-        s_shift[c] = p.beta[c] - (float)mean * p.gamma[c] * rstd;
+        bn_scale_shift(p.gamma[c], p.beta[c], (float)mean, rstd, s_scale[c], s_shift[c]);
         if (blockIdx.x == 0) {
             p.save_mean[c] = (float)mean;
             p.save_rstd[c] = rstd;
@@ -210,8 +218,7 @@ __global__ void __launch_bounds__(BT, MINB) bn_act_bwd_reduce_kernel(const uint4
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
         const int c = chunk * 8 + i;
-        sc[i] = p.gamma[c] * p.save_rstd[c];
-        sh[i] = p.beta[c] - p.save_mean[c] * sc[i];
+        bn_scale_shift(p.gamma[c], p.beta[c], p.save_mean[c], p.save_rstd[c], sc[i], sh[i]);
     }
     // packed fp32x2 arithmetic (FFMA2 / FMUL2 / FADD2, IEEE per lane: the same values as the scalar form): a bf16x2 pair
     // converts straight into a float2 and the five arithmetic instructions per element become five per pair
@@ -261,8 +268,7 @@ __global__ void __launch_bounds__(BT, MINB) bn_act_bwd_kernel(const uint4* __res
         const double mean = (double)p.save_mean[c], rstd = (double)p.save_rstd[c], ga = (double)p.gamma[c];
         const double sg = p.sum[c], sgx = rstd * (p.sumsq[c] - mean * sg);      // sum(g'), sum(g' * xhat)
         const double A = ga * rstd, mg = sg * invn, mgx = sgx * invn;
-        s_A[c] = (float)A;
-        s_sh[c] = (float)((double)p.beta[c] - mean * A);
+        bn_scale_shift(p.gamma[c], p.beta[c], p.save_mean[c], p.save_rstd[c], s_A[c], s_sh[c]);   // (float)A == s_A[c]
         s_B[c] = (float)(-A * rstd * mgx);
         s_C[c] = (float)(A * (mean * rstd * mgx - mg));
         if (blockIdx.x == 0 && p.dgamma_accum != nullptr) {   // d gamma = sum(g' * xhat), d beta = sum(g'): add to .grad
