@@ -423,6 +423,28 @@ int uaps_grad_reduce_adam(float* p, const float* const* grads, float* m, float* 
 int uaps_confusion(const float* logits, const int64_t* labels, int B, int C, int64_t HW, uint64_t* conf,
                    cudaStream_t stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Validation head: one validation batch of UAPS_train.py:377-385 (main decoder's logits -> CrossEntropyLoss() with
+ * torch's default ignore_index -100, and the confusion matrix behind utilities/metrics.py), appended as one row of an
+ * epoch table that stays on the device until the epoch ends.
+ *   uaps_val_counts: reads logits [B,C,HW] fp32 and labels [B,HW] int64 once; per pixel pred = argmax(softmax(z))
+ *     (bit-exact with torch, as uaps_confusion) and the fp32 term -log_softmax(z)[y].  A label of -100 is left out of the
+ *     CE and the counts (it still counts as a pixel); any other label outside [0, C) is counted as BAD.  Per-block partial
+ *     sums go to `workspace` (>= uaps_val_workspace_bytes(C, B, HW) bytes, 8-byte aligned, no initialisation needed).
+ *   uaps_val_fold: one block adds those partials in a fixed order (bitwise reproducible) and writes row r = state[0] of
+ *     table[max_batches][C*C + 3] (fp64): C*C counts (row = label, column = prediction) | CE sum over the non-ignored
+ *     pixels | non-ignored pixels | pixels (B*HW); then state[0] = r + 1.  If r >= max_batches nothing is written and
+ *     state[1] = 1 (overflow).  state[2] += the batch's bad labels.  state: 3 uint32, zeroed by the caller per table.
+ * Same (B, C, HW) and workspace in both calls.  Both only read and write device memory at addresses fixed by their
+ * arguments, so the pair can be captured into a CUDA graph: every replay appends the next row.
+ * Algorithmic HBM bytes per pixel: 4C (logits) + 8 (label) read.
+ * ------------------------------------------------------------------------------------------- */
+size_t uaps_val_workspace_bytes(int C, int B, int64_t HW);
+int uaps_val_counts(const float* logits, const int64_t* labels, int B, int C, int64_t HW, void* workspace,
+                    size_t workspace_bytes, cudaStream_t stream);
+int uaps_val_fold(const void* workspace, size_t workspace_bytes, int B, int C, int64_t HW, double* table,
+                  int max_batches, uint32_t* state, cudaStream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -90,6 +90,9 @@ _SIGNATURES = {
     "uaps_conv_wgrad": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, C.c_size_t, _vp]),
     "uaps_adam_step": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _f, _f, _f, _f, _f, _vp, _vp, _vp]),
     "uaps_confusion": (_i, [_vp, _vp, _i, _i, _i64, _vp, _vp]),
+    "uaps_val_workspace_bytes": (C.c_size_t, [_i, _i, _i64]),
+    "uaps_val_counts": (_i, [_vp, _vp, _i, _i, _i64, _vp, C.c_size_t, _vp]),
+    "uaps_val_fold": (_i, [_vp, C.c_size_t, _i, _i, _i64, _vp, _i, _vp, _vp]),
     "uaps_peer_alloc": (_i, [_vp, C.c_size_t]),
     "uaps_peer_free": (_i, [_vp]),
     "uaps_grad_reduce_adam": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i, _i, _i64, _f, _f, _f, _f, _f, _vp, _vp, _vp]),

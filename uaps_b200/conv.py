@@ -101,19 +101,34 @@ class PackedConv:
         else:
             self.cout = co
             self.cin1, self.cin2 = (ci, 0) if cin_split is None else (cin_split, ci - cin_split)
-        self.ks, self.fold = ks, fold
+        self.ks, self.fold, self.transpose, self.shape = ks, fold, transpose, tuple(w.shape)
         nbytes = L.lib().uaps_conv_packed_bytes(self.cout, self.cin1, self.cin2, ks, fold)
         if nbytes == 0:
             raise RuntimeError("unsupported convolution shape")
         self.packed = torch.empty(nbytes, dtype=torch.uint8, device=w.device)
-        with L.on_device(w.device):
-            L.check(L.lib().uaps_conv_pack_weights(w.data_ptr(), self.packed.data_ptr(), self.cout, self.cin1, self.cin2,
-                                                   ks, int(transpose), fold, L.stream_ptr()), "uaps_conv_pack_weights")
+        self._pack(w)
         self.bias = None if bias is None else bias.detach().float().contiguous()
         if self.bias is not None and fold > 1:                # virtual bias: one padded copy per sub-pixel
             b = torch.zeros(pad16(self.cout), dtype=torch.float32, device=w.device)
             b[:self.cout] = self.bias
             self.bias = b.repeat(fold).contiguous()
+
+    def _pack(self, w: torch.Tensor) -> None:
+        with L.on_device(w.device):
+            L.check(L.lib().uaps_conv_pack_weights(w.data_ptr(), self.packed.data_ptr(), self.cout, self.cin1, self.cin2,
+                                                   self.ks, int(self.transpose), self.fold, L.stream_ptr()),
+                    "uaps_conv_pack_weights")
+
+    def repack(self, weight: torch.Tensor, bias: Optional[torch.Tensor]) -> "PackedConv":
+        """Pack new weights of the same shape into this layer's existing buffers (weights re-packed, bias copied), so a
+        CUDA graph that reads them sees the new values on its next replay.  Unfolded layers (fold = 1) only."""
+        w = weight.detach().float().contiguous()
+        if tuple(w.shape) != self.shape or (bias is None) != (self.bias is None) or self.fold != 1:
+            raise RuntimeError("repack needs an unfolded layer and weights of the shape it was built with")
+        self._pack(w)
+        if bias is not None:
+            self.bias.copy_(bias.detach())
+        return self
 
     def __call__(self, x1: torch.Tensor, x2: Optional[torch.Tensor] = None, out_nchw_f32: bool = False,
                  split: int = 0, slope: float = 1.0, bn_sums: Optional[torch.Tensor] = None, bn_nrep: int = 0):

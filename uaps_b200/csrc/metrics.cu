@@ -1,32 +1,13 @@
 // On-device segmentation metrics (SURVEY.md 8(f2)): the confusion matrix behind utilities/metrics.py
 // (pixel_accuracy :8-13, mIoU :16-37, mDice :40-61) in one pass over the logits, so the training loop needs one
 // host sync per epoch instead of the reference's ~20 per iteration (UAPS_train.py:295-306).
-// pred = argmax(softmax(logits)) exactly as torch computes it (softmax rounding can merge two nearly equal
-// logits into a tie that argmax then resolves to the lower index, so the softmax chain is reproduced).
-#include "common.cuh"
+// pred = argmax(softmax(logits)) exactly as torch computes it (argmax_exact.cuh, shared with the validation head).
+#include "argmax_exact.cuh"
 
 namespace uaps {
 namespace {
 
 constexpr int MT = 256;
-
-template <int C>
-__device__ __forceinline__ int argmax_softmax(const float (&z)[C]) {
-    float m = z[0];
-#pragma unroll
-    for (int c = 1; c < C; ++c) m = fmaxf(m, z[c]);
-    float e[C], s = 0.f;
-#pragma unroll
-    for (int c = 0; c < C; ++c) { e[c] = expf(__fsub_rn(z[c], m)); s = __fadd_rn(s, e[c]); }
-    int y = 0;
-    float best = __fdiv_rn(e[0], s);
-#pragma unroll
-    for (int c = 1; c < C; ++c) {
-        const float p = __fdiv_rn(e[c], s);
-        if (p > best) { best = p; y = c; }
-    }
-    return y;
-}
 
 // conf[label][pred] += 1 for every pixel; labels outside [0, C) are ignored
 template <int C>

@@ -30,19 +30,23 @@ def metrics_from_confusion(conf: torch.Tensor, smooth: float = 1e-10, n_pixels: 
     """(pixel_accuracy, mIoU, mDice) as 0-dim device tensors, the reference's formulas: classes 1..C-1, classes
     absent from the labels skipped (np.nanmean), smooth 1e-10.  n_pixels: the accuracy's denominator -- the reference
     divides by ``mask.numel()`` (utilities/metrics.py:12), so a pixel whose label lies outside [0, C) (an ignore
-    index) counts as WRONG there; the confusion matrix does not hold such pixels, hence the explicit total."""
+    index) counts as WRONG there; the confusion matrix does not hold such pixels, hence the explicit total.
+    conf may also be a stack [..., C, C] of matrices (n_pixels then a number or a tensor of shape [...]); the results are
+    then tensors of shape [...], one value per matrix."""
     c = conf.double()
-    acc = c.diagonal().sum() / (c.sum() if n_pixels is None else float(n_pixels))
-    inter = c.diagonal()[1:]
-    label_n, pred_n = c.sum(1)[1:], c.sum(0)[1:]
+    diag = c.diagonal(dim1=-2, dim2=-1)
+    acc = diag.sum(-1) / (c.sum((-2, -1)) if n_pixels is None else
+                          (n_pixels.double() if torch.is_tensor(n_pixels) else float(n_pixels)))
+    inter = diag[..., 1:]
+    label_n, pred_n = c.sum(-1)[..., 1:], c.sum(-2)[..., 1:]
     union = label_n + pred_n - inter
     present = label_n > 0
     iou = (inter + smooth) / (union + smooth)
     dice = 2 * (inter + smooth) / (union + inter + smooth)
-    n = present.sum()
+    n = present.sum(-1)
     nan = torch.full((), float("nan"), dtype=torch.float64, device=conf.device)
-    miou = torch.where(n > 0, (iou * present).sum() / n.clamp(min=1), nan)
-    mdice = torch.where(n > 0, (dice * present).sum() / n.clamp(min=1), nan)
+    miou = torch.where(n > 0, (iou * present).sum(-1) / n.clamp(min=1), nan)
+    mdice = torch.where(n > 0, (dice * present).sum(-1) / n.clamp(min=1), nan)
     return acc, miou, mdice
 
 

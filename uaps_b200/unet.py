@@ -236,19 +236,28 @@ class UNet_UAPS(nn.Module):
         b = (conv.bias.detach().float() - bn.running_mean.detach().float()) * s + bn.bias.detach().float()
         return w.contiguous(), b.contiguous()
 
-    def _block_plan(self, blk, cin_split=None):
+    def _block_plan(self, blk, cin_split=None, make=PackedConv):
         cc = blk.conv_conv
         w0, b0 = self._fold_bn(cc.get_submodule("0"), cc.get_submodule("1"))
         w4, b4 = self._fold_bn(cc.get_submodule("4"), cc.get_submodule("5"))
-        return PackedConv(w0, b0, cin_split=cin_split), PackedConv(w4, b4)
+        return make(w0, b0, cin_split=cin_split), make(w4, b4)
 
-    def _decoder_plan(self, dm: nn.Module):
+    def _decoder_plan(self, dm: nn.Module, make=PackedConv):
         dec = []
         for i in range(1, 5):
             up = dm.get_submodule(f"up{i}")
             c2 = FT_CHNS[4 - i]
-            dec.append((PackedConv(up.conv1x1.weight, up.conv1x1.bias), *self._block_plan(up.conv, cin_split=c2)))
-        return dec, PackedConv(dm.out_conv.weight, dm.out_conv.bias)
+            dec.append((make(up.conv1x1.weight, up.conv1x1.bias), *self._block_plan(up.conv, cin_split=c2, make=make)))
+        return dec, make(dm.out_conv.weight, dm.out_conv.bias)
+
+    def _main_plan(self, make=PackedConv):
+        """(enc, dec, out): the BN-folded layers of encoder + main decoder, each built by ``make(weight, bias,
+        cin_split=None)`` in a fixed order (``validate.Validator`` re-packs its own copy in place through it)."""
+        enc = [self._block_plan(self.encoder.in_conv, make=make)] + \
+              [self._block_plan(self.encoder.get_submodule(f"down{lvl}").maxpool_conv.get_submodule("1"), make=make)
+               for lvl in range(1, 5)]
+        dec, out = self._decoder_plan(self.main_decoder, make=make)
+        return enc, dec, out
 
     def _inference_plan(self):
         """Packed, BN-folded layers of encoder + main decoder (built lazily, dropped by train() / load_state_dict()), and
@@ -256,10 +265,7 @@ class UNet_UAPS(nn.Module):
         plan = getattr(self, "_infer_plan", None)
         if plan is not None:
             return plan
-        enc = [self._block_plan(self.encoder.in_conv)] + \
-              [self._block_plan(self.encoder.get_submodule(f"down{lvl}").maxpool_conv.get_submodule("1")) for lvl in range(1, 5)]
-        dec, out = self._decoder_plan(self.main_decoder)
-        self._infer_plan = (enc, dec, out, {})
+        self._infer_plan = (*self._main_plan(), {})
         return self._infer_plan
 
     def _aux_plan(self, a: int):
