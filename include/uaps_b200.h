@@ -445,6 +445,47 @@ int uaps_val_counts(const float* logits, const int64_t* labels, int B, int C, in
 int uaps_val_fold(const void* workspace, size_t workspace_bytes, int B, int C, int64_t HW, double* table,
                   int max_batches, uint32_t* state, cudaStream_t stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Whole-network inference: the eval-mode forward of UNet_UAPS's encoder + main decoder (UAPS_unet.py:224-226, the
+ * output UAPS_train.py:377 and UAPS-Testing.ipynb use) without PyTorch -- the result of UNet_UAPS.predict in eval mode,
+ * bit for bit.  in_chns in 1..16, C (classes) in 2..UAPS_CMAX.  Auxiliary decoders are not part of it.
+ *
+ * Parameter blob: fp32, uaps_unet_params_count(in_chns, C) values, the encoder.* then main_decoder.* tensors of the
+ * reference state_dict in state_dict order, each flattened, num_batches_tracked left out:
+ *   encoder.in_conv, encoder.down1 .. down4 (ConvBlock): per block conv_conv.0 weight, bias | conv_conv.1 (BatchNorm)
+ *     weight, bias, running_mean, running_var | conv_conv.4 weight, bias | conv_conv.5 weight, bias, running_mean,
+ *     running_var;
+ *   main_decoder.up1 .. up4: conv1x1 weight, bias, then its ConvBlock `conv` as above;
+ *   main_decoder.out_conv weight, bias.
+ * (uaps_b200.unet.inference_params builds it from a model or a checkpoint's state_dict.)
+ *
+ * uaps_unet_infer_prepare folds each BatchNorm's running statistics into the conv before it, with the roundings of
+ * UNet_UAPS._fold_bn (s = gamma * rsqrtf(var + 1e-5); w * s; (b - mean) * s + beta; every op rounded on its own), and
+ * packs the 23 layers for the tcgen05 convolution: two launches, no host synchronisation, capturable.  `state`:
+ * >= uaps_unet_infer_state_bytes(in_chns, C) bytes of device memory, 16-byte aligned, owned by the caller; the blob
+ * is only read during the call's launches, so it may be freed once they have run.  Re-run prepare after new weights.
+ *
+ * uaps_unet_infer_run: x [B, in_chns, H, W] fp32 NCHW (16-byte aligned), H and W multiples of 16; writes
+ *   logits [B, C, H, W] fp32 (nullable, 16-byte aligned) and labels [B, H, W] uint8 (nullable, 4-byte aligned) =
+ *   argmax_c softmax(logits) with torch's rounding and tie rule (lowest index), i.e. torch.softmax(z, 1).argmax(1).
+ *   At least one of the two.  workspace: >= uaps_unet_infer_workspace_bytes(in_chns, C, B, H, W) bytes, 16-byte
+ *   aligned, no initialisation needed (about 126 bytes per pixel of the batch).  The launch sequence depends on the
+ *   arguments only, so the call can be captured into a CUDA graph and replayed (also across a later prepare into the
+ *   same state).  Calls that share a workspace must be ordered.
+ * uaps_unet_infer_layer: byte offsets inside `state` of layer `layer` (0..22, UNet_UAPS._main_plan order: the encoder's
+ *   ten convs, then per decoder level conv1x1 and the two block convs, then out_conv) -- its folded fp32 weight
+ *   [cout][cin][ks][ks] and bias [cout], and its packed weights (packed_bytes bytes), for inspection.
+ * The size queries return 0 for arguments outside the supported range.
+ * ------------------------------------------------------------------------------------------- */
+size_t uaps_unet_params_count(int in_chns, int C);
+size_t uaps_unet_infer_state_bytes(int in_chns, int C);
+size_t uaps_unet_infer_workspace_bytes(int in_chns, int C, int B, int H, int W);
+int uaps_unet_infer_prepare(const float* params, int in_chns, int C, void* state, size_t state_bytes, cudaStream_t stream);
+int uaps_unet_infer_run(const void* state, size_t state_bytes, int in_chns, int C, const float* x, int B, int H, int W,
+                        void* workspace, size_t workspace_bytes, float* logits, uint8_t* labels, cudaStream_t stream);
+int uaps_unet_infer_layer(int in_chns, int C, int layer, size_t* weight_offset, size_t* bias_offset,
+                          size_t* packed_offset, size_t* packed_bytes);
+
 #ifdef __cplusplus
 }
 #endif

@@ -97,6 +97,12 @@ _SIGNATURES = {
     "uaps_peer_free": (_i, [_vp]),
     "uaps_grad_reduce_adam": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i, _i, _i64, _f, _f, _f, _f, _f, _vp, _vp, _vp]),
     "uaps_perturb3_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _u64, _f, _d, _vp, _vp, _f, _vp, _i, _i, _i64, _vp]),
+    "uaps_unet_params_count": (C.c_size_t, [_i, _i]),
+    "uaps_unet_infer_state_bytes": (C.c_size_t, [_i, _i]),
+    "uaps_unet_infer_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i]),
+    "uaps_unet_infer_prepare": (_i, [_vp, _i, _i, _vp, C.c_size_t, _vp]),
+    "uaps_unet_infer_run": (_i, [_vp, C.c_size_t, _i, _i, _vp, _i, _i, _i, _vp, C.c_size_t, _vp, _vp, _vp]),
+    "uaps_unet_infer_layer": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -506,6 +506,29 @@ def load_reference_state_dict(model: nn.Module, state_dict: Dict[str, torch.Tens
     return model.load_state_dict(cleaned, strict=strict)
 
 
+def inference_params(model_or_state_dict) -> torch.Tensor:
+    """The parameter blob of the C inference entry points (``uaps_unet_infer_prepare``, include/uaps_b200.h): the
+    ``encoder.*`` and ``main_decoder.*`` tensors of the state_dict in state_dict order, without ``num_batches_tracked``,
+    flattened into one contiguous fp32 tensor on the tensors' device.  Takes a model or a state_dict, with or without the
+    ``module.`` prefix of a reference checkpoint."""
+    sd = model_or_state_dict.state_dict() if isinstance(model_or_state_dict, nn.Module) else model_or_state_dict
+    sd = {(k[len("module."):] if k.startswith("module.") else k): v for k, v in sd.items()}
+    parts = [v.detach().reshape(-1).float() for k, v in sd.items()
+             if k.startswith(("encoder.", "main_decoder.")) and not k.endswith("num_batches_tracked")]
+    try:
+        in_chns = sd["encoder.in_conv.conv_conv.0.weight"].shape[1]
+        C = sd["main_decoder.out_conv.weight"].shape[0]
+    except KeyError as e:
+        raise ValueError(f"not a UNet_UAPS state_dict: {e} is missing") from None
+    from . import _lib as L
+    blob = torch.cat(parts)
+    want = L.lib().uaps_unet_params_count(in_chns, C)
+    if blob.numel() != want:
+        raise ValueError(f"parameter blob of {blob.numel()} values, the network ({in_chns} input channels, {C} classes) "
+                         f"needs {want}")
+    return blob
+
+
 def save_checkpoint(path: str, model: nn.Module, optimizer, epoch: int, best_dice: float, data_parallel_keys: bool = True):
     """The reference's checkpoint dict (UAPS_train.py:443-450): {"epoch", "best_dice_1", "state_dict", "optimizer"},
     with the ``module.`` key prefix its DataParallel wrapper produces, so the reference's notebooks can load it."""
