@@ -448,7 +448,8 @@ int uaps_val_fold(const void* workspace, size_t workspace_bytes, int B, int C, i
 /* ---------------------------------------------------------------------------------------------
  * Whole-network inference: the eval-mode forward of UNet_UAPS's encoder + main decoder (UAPS_unet.py:224-226, the
  * output UAPS_train.py:377 and UAPS-Testing.ipynb use) without PyTorch -- the result of UNet_UAPS.predict in eval mode,
- * bit for bit.  in_chns in 1..16, C (classes) in 2..UAPS_CMAX.  Auxiliary decoders are not part of it.
+ * bit for bit.  in_chns in 1..16, C (classes) in 2..UAPS_CMAX.  Auxiliary decoders are not part of it (the ensemble
+ * entry points below run them).
  *
  * Parameter blob: fp32, uaps_unet_params_count(in_chns, C) values, the encoder.* then main_decoder.* tensors of the
  * reference state_dict in state_dict order, each flattened, num_batches_tracked left out:
@@ -485,6 +486,52 @@ int uaps_unet_infer_run(const void* state, size_t state_bytes, int in_chns, int 
                         void* workspace, size_t workspace_bytes, float* logits, uint8_t* labels, cudaStream_t stream);
 int uaps_unet_infer_layer(int in_chns, int C, int layer, size_t* weight_offset, size_t* bias_offset,
                           size_t* packed_offset, size_t* packed_bytes);
+
+/* ---------------------------------------------------------------------------------------------
+ * Ensemble uncertainty inference: every decoder of UNet_UAPS, the auxiliary decoders' perturbations and the ensemble
+ * head above, without PyTorch -- the result of UNet_UAPS.predict_uncertainty(x, seed=...) in eval mode, bit for bit
+ * (UAPS-Testing.ipynb cell 11).  in_chns in 1..16, C in 2..UAPS_CMAX, n_aux (auxiliary decoders) in 1..UAPS_KMAX - 1,
+ * so K = 1 + n_aux decoders.
+ *
+ * Parameter blob: fp32, uaps_unet_ensemble_params_count(in_chns, C, n_aux) values: the blob of uaps_unet_params_count
+ * followed by the aux_decoder1.* .. aux_decoder<n_aux>.* tensors, each laid out as main_decoder.* (state_dict order,
+ * num_batches_tracked left out; uaps_b200.unet.inference_params(..., ensemble=True) builds it).  The network has
+ * 23 + 13 * n_aux layers: those of uaps_unet_infer_layer, then per auxiliary decoder its 13 in the same order.
+ *
+ * uaps_unet_ensemble_prepare: as uaps_unet_infer_prepare, for all layers (two launches, no host synchronisation,
+ *   capturable); `state`: >= uaps_unet_ensemble_state_bytes(in_chns, C, n_aux) bytes, 16-byte aligned.
+ *
+ * Random draws: `draws` is device int64 [2][uaps_unet_ensemble_draws_count(n_aux)] (8-byte aligned), one column per
+ *   perturbation launch, exactly as UNet_UAPS._ensemble_draws lays it out: row 0 the Philox keys, row 1 the
+ *   FeatureDropout threshold u as fp32 in the low 4 bytes (little-endian).  Columns 0-4: levels 0-4 of the launch shared
+ *   by auxiliary decoders 1-3 (FeatureNoise, Dropout(0.5), FeatureDropout); 5-9: decoder 4's fresh FeatureNoise draw;
+ *   10-14: decoder 5's fresh Dropout draw.  u is expected in [0.7, 0.9] (UAPS_unet.py:165); the kernels do not check it.
+ *   The draws are read only by the kernels, so a caller may write new ones between replays of a captured graph.
+ *
+ * uaps_unet_ensemble_run: x [B, in_chns, H, W] fp32 NCHW (16-byte aligned), H and W multiples of 16.  Writes, as
+ *   uaps_ensemble_head over the K decoders' logits (main decoder first): labels [B, H, W] uint8 (required, 4-byte
+ *   aligned), uncertainty [B, H, W], image_uncertainty [B] and mean_prob [B, C, H, W] fp32 (each nullable, 16-byte
+ *   aligned: the head's vector width, and with it the chunking of the per-image fp64 sum, follows the alignment).
+ *   workspace: >= uaps_unet_ensemble_workspace_bytes(in_chns, C, n_aux, B, H, W) bytes, 16-byte aligned, no
+ *   initialisation needed: about 126 + 62 * min(n_aux, 3) + 4 * C * (1 + n_aux) bytes per pixel of the batch, plus 4
+ *   for n_aux >= 3 (380 at C = 4, n_aux = 3).  Every argument is checked before the first launch and the launch
+ *   sequence depends on the arguments only, so the call can be captured into a CUDA graph and replayed (also across a
+ *   later prepare into the same state, or new draws in the same buffer).  Calls that share a workspace must be ordered.
+ * uaps_unet_ensemble_layer: as uaps_unet_infer_layer for layer 0 .. 22 + 13 * n_aux.
+ * The size queries return 0 for arguments outside the supported range.
+ * ------------------------------------------------------------------------------------------- */
+size_t uaps_unet_ensemble_params_count(int in_chns, int C, int n_aux);
+size_t uaps_unet_ensemble_state_bytes(int in_chns, int C, int n_aux);
+size_t uaps_unet_ensemble_draws_count(int n_aux);               /* 5 * (1 + max(0, n_aux - 3)) */
+size_t uaps_unet_ensemble_workspace_bytes(int in_chns, int C, int n_aux, int B, int H, int W);
+int uaps_unet_ensemble_prepare(const float* params, int in_chns, int C, int n_aux, void* state, size_t state_bytes,
+                               cudaStream_t stream);
+int uaps_unet_ensemble_run(const void* state, size_t state_bytes, int in_chns, int C, int n_aux, const float* x,
+                           int B, int H, int W, const int64_t* draws, void* workspace, size_t workspace_bytes,
+                           uint8_t* labels, float* uncertainty, float* image_uncertainty, float* mean_prob,
+                           cudaStream_t stream);
+int uaps_unet_ensemble_layer(int in_chns, int C, int n_aux, int layer, size_t* weight_offset, size_t* bias_offset,
+                             size_t* packed_offset, size_t* packed_bytes);
 
 #ifdef __cplusplus
 }

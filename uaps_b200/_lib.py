@@ -103,6 +103,14 @@ _SIGNATURES = {
     "uaps_unet_infer_prepare": (_i, [_vp, _i, _i, _vp, C.c_size_t, _vp]),
     "uaps_unet_infer_run": (_i, [_vp, C.c_size_t, _i, _i, _vp, _i, _i, _i, _vp, C.c_size_t, _vp, _vp, _vp]),
     "uaps_unet_infer_layer": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp]),
+    "uaps_unet_ensemble_params_count": (C.c_size_t, [_i, _i, _i]),
+    "uaps_unet_ensemble_state_bytes": (C.c_size_t, [_i, _i, _i]),
+    "uaps_unet_ensemble_draws_count": (C.c_size_t, [_i]),
+    "uaps_unet_ensemble_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i, _i, _i]),
+    "uaps_unet_ensemble_prepare": (_i, [_vp, _i, _i, _i, _vp, C.c_size_t, _vp]),
+    "uaps_unet_ensemble_run": (_i, [_vp, C.c_size_t, _i, _i, _i, _vp, _i, _i, _i, _vp, _vp, C.c_size_t, _vp, _vp, _vp, _vp,
+                                    _vp]),
+    "uaps_unet_ensemble_layer": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -18,6 +18,7 @@ bilinear(align_corners=True) because ``UpBlock``'s ``bilinear=True`` default win
 """
 from __future__ import annotations
 
+import re
 from typing import Dict, List, Optional, Sequence
 
 import numpy as np
@@ -506,15 +507,26 @@ def load_reference_state_dict(model: nn.Module, state_dict: Dict[str, torch.Tens
     return model.load_state_dict(cleaned, strict=strict)
 
 
-def inference_params(model_or_state_dict) -> torch.Tensor:
+def inference_params(model_or_state_dict, *, ensemble: bool = False) -> torch.Tensor:
     """The parameter blob of the C inference entry points (``uaps_unet_infer_prepare``, include/uaps_b200.h): the
     ``encoder.*`` and ``main_decoder.*`` tensors of the state_dict in state_dict order, without ``num_batches_tracked``,
     flattened into one contiguous fp32 tensor on the tensors' device.  Takes a model or a state_dict, with or without the
-    ``module.`` prefix of a reference checkpoint."""
+    ``module.`` prefix of a reference checkpoint.
+
+    ``ensemble=True``: the blob of ``uaps_unet_ensemble_prepare`` -- the same, followed by every ``aux_decoderN.*``
+    tensor (N = 1 .. n_aux, state_dict order).  n_aux is read from the keys; it must be 1..5 with no gap."""
     sd = model_or_state_dict.state_dict() if isinstance(model_or_state_dict, nn.Module) else model_or_state_dict
     sd = {(k[len("module."):] if k.startswith("module.") else k): v for k, v in sd.items()}
+    prefixes = ("encoder.", "main_decoder.")
+    if ensemble:
+        found = sorted({int(m.group(1)) for k in sd if (m := re.match(r"aux_decoder(\d+)\.", k))})
+        n_aux = len(found)
+        if found != list(range(1, n_aux + 1)) or not 1 <= n_aux <= 5:
+            raise ValueError(f"the ensemble blob needs auxiliary decoders 1..n_aux with n_aux in 1..5; the state_dict has "
+                             f"{['aux_decoder%d' % a for a in found] or 'none'}")
+        prefixes += tuple(f"aux_decoder{a}." for a in found)
     parts = [v.detach().reshape(-1).float() for k, v in sd.items()
-             if k.startswith(("encoder.", "main_decoder.")) and not k.endswith("num_batches_tracked")]
+             if k.startswith(prefixes) and not k.endswith("num_batches_tracked")]
     try:
         in_chns = sd["encoder.in_conv.conv_conv.0.weight"].shape[1]
         C = sd["main_decoder.out_conv.weight"].shape[0]
@@ -522,10 +534,10 @@ def inference_params(model_or_state_dict) -> torch.Tensor:
         raise ValueError(f"not a UNet_UAPS state_dict: {e} is missing") from None
     from . import _lib as L
     blob = torch.cat(parts)
-    want = L.lib().uaps_unet_params_count(in_chns, C)
+    want = L.lib().uaps_unet_ensemble_params_count(in_chns, C, n_aux) if ensemble else L.lib().uaps_unet_params_count(in_chns, C)
     if blob.numel() != want:
-        raise ValueError(f"parameter blob of {blob.numel()} values, the network ({in_chns} input channels, {C} classes) "
-                         f"needs {want}")
+        what = f"{in_chns} input channels, {C} classes" + (f", {n_aux} auxiliary decoders" if ensemble else "")
+        raise ValueError(f"parameter blob of {blob.numel()} values, the network ({what}) needs {want}")
     return blob
 
 
