@@ -49,6 +49,33 @@ def test_closed_form_backward_matches_golden(loss_cases):
         assert cf["l_uncert"].item() == pytest.approx(float(c["l_uncert"]), rel=1e-5)
 
 
+@pytest.mark.parametrize("every", [True, False])
+@pytest.mark.parametrize("margin", [60.0, 95.0, 110.0, 300.0, 700.0])
+def test_closed_form_matches_fp64_autograd_at_large_margins(margin, every):
+    """The GPU loss tests take the fp64 closed form as the gradient reference where fp32 autograd of the oracle is NaN
+    (a class more than ~104 nats below the max in every decoder: q_c = 0 and d xlogy(q, q)/dq = -inf).  In fp64, q_c
+    stays positive up to ~745 nats, so autograd of the same oracle is finite there and the closed form must equal it."""
+    K, C, B, H, W = 3, 4, 2, 4, 6
+    g = torch.Generator().manual_seed(17)
+    z = [torch.randn(B, C, H, W, generator=g, dtype=torch.float64) * 2 for _ in range(K)]
+    pix = torch.arange(B * H * W).view(B, H, W) % 3 == 0
+    for k in range(K if every else 1):                    # classes 2 and 3 `margin` nats below the max
+        top = z[k][:, :2].amax(1)
+        for c in (2, 3):
+            z[k][:, c] = torch.where(pix, top - margin, z[k][:, c])
+    mix_w = [0.5, 0.3, 0.2]
+    zr = [t.clone().requires_grad_(True) for t in z]
+    ref = unlabeled_loss_ref(zr, mix_w, 0.3, 0.2)
+    ref["loss_u"].backward()
+    auto = torch.stack([t.grad for t in zr])
+    cf = unlabeled_loss_fp64_closed_form(z, mix_w, 0.3, 0.2, ref["pseudo"])
+    dz = torch.stack(cf["dz"])
+    assert torch.isfinite(auto).all() and torch.isfinite(dz).all()
+    assert (dz - auto).abs().max().item() <= 1e-9 * auto.abs().max().item()
+    assert cf["ps_loss"].item() == pytest.approx(ref["ps_loss"].item(), rel=1e-12)
+    assert cf["l_uncert"].item() == pytest.approx(ref["l_uncert"].item(), rel=1e-12)
+
+
 def test_ties_take_lowest_index(loss_cases):
     c = loss_cases["k4c4_ties"]
     # planes 1 == 0 and 3 == 2 in every decoder, so only labels 0 and 2 can win

@@ -85,7 +85,7 @@ struct PixelState {
     float p[K][C];   // softmax
     float l[K][C];   // log-softmax / U
     float q[C];      // mean prediction
-    float lq[C];     // log q / U  (-inf when q == 0)
+    float lq[C];     // log q / U  (0 for q == 0 after kl_terms<GUARD>; see there)
     float V[K];      // KL(q || p_k) summed over classes
     float E[K];      // exp(-V)
     int y;           // pseudo-label / label
@@ -231,7 +231,10 @@ __device__ __noinline__ int argmax_exact_gmem(const Args& a, size_t pix_off) {
 }
 
 // mean prediction (UAPS_train.py:223) and KL maps (:226-236): V_k = sum_c xlogy(q,q) - q * l_kc, E_k = exp(-V_k).
-// GUARD: apply xlogy's q == 0 -> 0 rule explicitly (the fast path leaves it to the NaN check of its caller).
+// GUARD: apply xlogy's q == 0 -> 0 rule explicitly (the fast path leaves it to the NaN check of its caller), and give
+// such a q a finite log, lq = 0.  lq is read again only by pass 2, in Gq_c, which enters dz only multiplied by p_kc
+// <= K q_c: a -inf there made the pixel's dz NaN (0 * inf) where the limit is finite.  The default arithmetic's
+// lg2.approx.ftz also flushes a subnormal q to -inf, so there the rule covers q < FLT_MIN (terms below 1e-36).
 template <int K, int C, bool EXACT, bool GUARD>
 __device__ __forceinline__ void kl_terms(PixelState<K, C>& st) {
     constexpr float U = LogUnit<EXACT>::U;
@@ -243,9 +246,14 @@ __device__ __forceinline__ void kl_terms(PixelState<K, C>& st) {
         for (int k = 1; k < K; ++k) acc = __fadd_rn(acc, st.p[k][c]);
         const float q = acc * (1.0f / K);
         st.q[c] = q;
-        st.lq[c] = EXACT ? logf(q) : lg2_approx(q);
-        if constexpr (GUARD) h += (q == 0.f) ? 0.f : q * st.lq[c];
-        else h = fmaf(q, st.lq[c], h);
+        if constexpr (GUARD) {
+            const bool zero = EXACT ? q == 0.f : q < 1.17549435e-38f;
+            st.lq[c] = zero ? 0.f : (EXACT ? logf(q) : lg2_approx(q));
+            h += zero ? 0.f : q * st.lq[c];
+        } else {
+            st.lq[c] = EXACT ? logf(q) : lg2_approx(q);
+            h = fmaf(q, st.lq[c], h);
+        }
     }
 #pragma unroll
     for (int k = 0; k < K; ++k) {
