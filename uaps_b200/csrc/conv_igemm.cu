@@ -1399,6 +1399,9 @@ int conv_fprop_impl(const void* x1, int c1_stride, const void* x2, int c2_stride
             if (smem > 227 * 1024) return UAPS_ERANGE;
             long long gridx = (long long)device_info().sm_count * per_sm;
             if (gridx > a.num_tiles) gridx = a.num_tiles;
+            if (getenv("UAPS_CONV_DEBUG") != nullptr)
+                fprintf(stderr, "conv_sn_small<%d,%d>: per_sm %d stages %d smem %zu units %d\n", pl.ck, cout_real, per_sm, stages,
+                        smem, a.num_tiles);
             cudaError_t e;
 #define UAPS_CONV_LAUNCH4(CKV, CV)                                                                                          \
             e = cudaFuncSetAttribute(conv_sn_small_kernel<CKV, CV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   \
@@ -1527,7 +1530,10 @@ int conv_fprop_impl(const void* x1, int c1_stride, const void* x2, int c2_stride
             gridx = gridx / pl.n_tiles * pl.n_tiles;
             if (gridx < pl.n_tiles) gridx = pl.n_tiles;
         }
-#define UAPS_CONV_LAUNCH2(CKV)                                                                                             \
+        if (getenv("UAPS_CONV_DEBUG") != nullptr)
+            fprintf(stderr, "conv_persistent<%d>: per_sm %d stages %d smem %zu grid %lld num_tiles %d\n", pl.ck, per_sm, stages,
+                    smem, gridx, a.num_tiles);
+#define UAPS_CONV_LAUNCH2(CKV)                                                                                           \
         e = cudaFuncSetAttribute(conv_igemm_persistent_kernel<CKV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   \
         if (e != cudaSuccess) return (int)e;                                                                                   \
         UAPS_LAUNCH(conv_igemm_persistent_kernel<CKV>, dim3((unsigned)gridx), dim3(THREADS2), smem, stream, m0, m1, a);

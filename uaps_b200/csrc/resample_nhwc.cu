@@ -229,6 +229,11 @@ __global__ void __launch_bounds__(RT) nchw_f32_to_nhwc_bf16_sums_kernel(const fl
     }
 }
 
+// torch's max-pool rule (nn.MaxPool2d on CUDA): scanning the window in (row, column) order, a candidate replaces the running
+// maximum when it is greater OR NaN -- so a NaN anywhere in the window propagates to the output (fmaxf would drop it, and a NaN
+// activation would vanish at the pooling layer instead of reaching the loss)
+__device__ __forceinline__ float pool_pick(float m, float v) { return (v > m || isnan(v)) ? v : m; }
+
 __global__ void __launch_bounds__(RT) maxpool2_fwd_kernel(const uint4* __restrict__ x, uint4* __restrict__ y, int B, int H, int W, int G) {
     grid_dep_launch();
     grid_dep_wait();
@@ -245,12 +250,13 @@ __global__ void __launch_bounds__(RT) maxpool2_fwd_kernel(const uint4* __restric
         unpack8(__ldg(xb), a); unpack8(__ldg(xb + G), c);
         unpack8(__ldg(xb + (size_t)W * G), d); unpack8(__ldg(xb + (size_t)W * G + G), e);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) a[i] = fmaxf(fmaxf(a[i], c[i]), fmaxf(d[i], e[i]));
+        for (int i = 0; i < 8; ++i) a[i] = pool_pick(pool_pick(pool_pick(a[i], c[i]), d[i]), e[i]);
         y[t] = pack8(a);
     }
 }
 
-// the gradient goes to the first maximum of the window in (row, column) order, as torch's max_pool2d backward does
+// the gradient goes to the element the forward picked (pool_pick in (row, column) order: the first maximum, or the last NaN),
+// as torch's max_pool2d backward does
 __global__ void __launch_bounds__(RT) maxpool2_bwd_kernel(const uint4* __restrict__ x, const uint4* __restrict__ gy,
                                                           uint4* __restrict__ gx, int B, int H, int W, int G) {
     grid_dep_launch();
@@ -275,7 +281,7 @@ __global__ void __launch_bounds__(RT) maxpool2_bwd_kernel(const uint4* __restric
             float m = v[0][i];
 #pragma unroll
             for (int k = 1; k < 4; ++k)
-                if (v[k][i] > m) { m = v[k][i]; best = k; }
+                if (v[k][i] > m || isnan(v[k][i])) { m = v[k][i]; best = k; }
 #pragma unroll
             for (int k = 0; k < 4; ++k) o[k][i] = (k == best) ? gv[i] : 0.f;
         }
