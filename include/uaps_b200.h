@@ -445,6 +445,15 @@ int uaps_val_counts(const float* logits, const int64_t* labels, int B, int C, in
 int uaps_val_fold(const void* workspace, size_t workspace_bytes, int B, int C, int64_t HW, double* table,
                   int max_batches, uint32_t* state, cudaStream_t stream);
 
+/* A second table row-aligned with the first: after uaps_val_fold has written row r = state[0] - 1, copies n fp32 device
+ * scalars, each read from its own address src[i] (src: host array of n device pointers, 1 <= n <=
+ * UAPS_VAL_SCALARS_MAX), to table[r][0..n-1] (fp64, table[max_rows][n]).  Nothing is written when state[1] (overflow)
+ * is set, state[0] == 0 or state[0] > max_rows.  One tiny launch; capturable like the pair above (the training log of
+ * UAPSTrainer: the iteration's losses beside the labeled batch's counts). */
+#define UAPS_VAL_SCALARS_MAX 16
+int uaps_val_scalars(const float* const* src, int n, double* table, int max_rows, const uint32_t* state,
+                     cudaStream_t stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Whole-network inference: the eval-mode forward of UNet_UAPS's encoder + main decoder (UAPS_unet.py:224-226, the
  * output UAPS_train.py:377 and UAPS-Testing.ipynb use) without PyTorch -- the result of UNet_UAPS.predict in eval mode,

@@ -2,6 +2,8 @@
 // decoder's logits in one read -- the confusion matrix behind pixel accuracy / mIoU / mDice (utilities/metrics.py) and
 // the cross-entropy sum of CrossEntropyLoss() (:75, ignore_index -100) -- then one fold that appends the batch as a row
 // of a caller-owned epoch table.  See include/uaps_b200.h for the contract and DESIGN.md f6 for the numbers.
+// uaps_val_scalars copies a few device scalars (a training iteration's losses, DESIGN.md f9) into the row of a second
+// table that the fold has just written, so the two tables stay row-aligned without the host.
 //
 // Grid as the ensemble head (ensemble_head.cu): blockIdx.y = image, blockIdx.x = a fixed span of that image's pixels.
 // The span is counted in pixels, so the number of blocks depends on (B, HW) only and uaps_val_fold can recompute it.
@@ -174,6 +176,19 @@ __global__ void __launch_bounds__(FOLD_THREADS) val_fold_kernel(const double* __
     }
 }
 
+struct ScalarSrc { const float* p[UAPS_VAL_SCALARS_MAX]; };
+
+// one warp: scalar i -> table[state[0] - 1][i], the row the preceding fold on the same state wrote
+__global__ void __launch_bounds__(kWarp) val_scalars_kernel(const __grid_constant__ ScalarSrc src, int n,
+                                                            double* __restrict__ table, unsigned max_rows,
+                                                            const uint32_t* __restrict__ state) {
+    grid_dep_launch();
+    grid_dep_wait();
+    const unsigned row = state[0];
+    if (state[1] != 0u || row == 0u || row > max_rows || (int)threadIdx.x >= n) return;   // overflow: nothing recorded
+    table[(size_t)(row - 1) * n + threadIdx.x] = (double)*src.p[threadIdx.x];
+}
+
 template <int C, int VEC>
 int launch_counts(CountArgs a, int B, cudaStream_t st) {
     a.groups_per_image = (unsigned)(a.HW / VEC);
@@ -250,5 +265,20 @@ UAPS_API int uaps_val_fold(const void* workspace, size_t workspace_bytes, int B,
     const uint32_t* words = reinterpret_cast<const uint32_t*>(ce + nblk);
     UAPS_LAUNCH(val::val_fold_kernel, dim3(1), dim3(val::FOLD_THREADS), 0, stream, ce, words, nblk, C,
                 (double)B * (double)HW, table, (unsigned)max_batches, state);
+    return UAPS_OK;
+}
+
+UAPS_API int uaps_val_scalars(const float* const* src, int n, double* table, int max_rows, const uint32_t* state,
+                              cudaStream_t stream) {
+    if (src == nullptr || table == nullptr || state == nullptr || max_rows < 0) return UAPS_EINVAL;
+    if (n < 1 || n > UAPS_VAL_SCALARS_MAX) return UAPS_ERANGE;
+    if (!aligned_to(table, 8) || !aligned_to(state, 4)) return UAPS_EALIGN;
+    val::ScalarSrc s{};
+    for (int i = 0; i < n; ++i) {
+        if (src[i] == nullptr) return UAPS_EINVAL;
+        if (!aligned_to(src[i], 4)) return UAPS_EALIGN;
+        s.p[i] = src[i];
+    }
+    UAPS_LAUNCH(val::val_scalars_kernel, dim3(1), dim3(kWarp), 0, stream, s, n, table, (unsigned)max_rows, state);
     return UAPS_OK;
 }

@@ -6,7 +6,8 @@ over one process per GPU.
 pseudo-label / KL-uncertainty / weighted CE+Dice loss (:223-277), the sigmoid ramp (:279-280), the
 total (:282), ``zero_grad / backward / Adam.step`` (:285-292) -- and returns the logged scalars as
 device tensors (the reference's nine ``.item()`` host syncs per iteration, :295-306, are left to
-the caller, once per epoch).
+the caller, once per epoch).  With ``UAPSConfig.train_log_rows > 0`` every iteration also appends those scalars and the
+labeled batch's confusion counts to a device-side training log, read once per epoch with ``log_result()``.
 
 Three ways to run the same iteration:
 
@@ -38,11 +39,19 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
+from . import _lib as L
 from . import perturb as P
 from .conv import WeightPacker, pack_scope
 from .stepctx import DeviceStepState, StepContext
 from .losses import uaps_supervised_loss, uaps_unlabeled_loss
 from .ramps import get_current_consistency_weight
+from .validate import append_row, finalize
+
+# the scalars of the training log, in the order of its columns (then loss_ce_k[0..K-1]): the names ``step`` returns
+LOG_SCALARS = ("loss", "supervised_loss", "total_loss_ce", "total_loss_dice", "ps_loss", "l_uncert")
+_LOG_ERRORS = {"ranks": "the ranks logged different numbers of training iterations",
+               "overflow": "more training iterations than UAPSConfig.train_log_rows since log_begin()",
+               "empty": "no training iteration logged since log_begin()"}
 
 
 @dataclass
@@ -59,6 +68,8 @@ class UAPSConfig:
     device_state: bool = True            # per-iteration scalars on the device (bf16 path only); False: host-drawn, by value
     cuda_graph: bool = True              # capture the device-state iteration into a CUDA graph (per input shape)
     graph_warmup: int = 2                # eager iterations of a shape before it is captured
+    train_log_rows: int = 0              # > 0: per-iteration training log on the device, this many iterations per epoch
+                                         # (UAPSTrainer.log_begin / log_result); 0: no log, no extra launches
 
 
 class FlatGradBuffer:
@@ -291,6 +302,17 @@ class UAPSTrainer:
             self.optimizer.attach_state(self.state)
             self.seed_rank = _mix64(self.cfg.seed, 0x52414E4B, self.rank)
             self.seed_shared = _mix64(self.cfg.seed, 0x53484152)
+        # ---- training log (DESIGN.md f9): one row per iteration, written inside the (captured) iteration -------------
+        rows = int(self.cfg.train_log_rows)
+        if rows < 0:
+            raise ValueError("train_log_rows must be >= 0")
+        self._log_ws: Dict[tuple, torch.Tensor] = {}
+        self.log_counts = self.log_state = self.log_scalars = None
+        if rows > 0:
+            C = getattr(model, "class_num", self.cfg.num_classes)
+            self.log_counts = torch.zeros((rows, C * C + 3), dtype=torch.float64, device=dev)   # uaps_val_fold's table
+            self.log_state = torch.zeros(3, dtype=torch.int32, device=dev)                      # rows, overflow, bad labels
+            self.log_scalars = torch.zeros((rows, len(LOG_SCALARS) + self.k), dtype=torch.float64, device=dev)
 
     # ---- iteration counter (drives the ramp, :279-280) ------------------------------------------------------
     @property
@@ -400,6 +422,8 @@ class UAPSTrainer:
             loss_u, ps_loss, l_unc, _, _ = uaps_unlabeled_loss(out_u, None, 0.0, 0.0, group=self.group,
                                                                step_state=st)                    # :223-280
             loss = sup + loss_u                                                                  # :282
+            if self.log_state is not None:
+                self._log_iteration(out_l[0], y_l, (loss, sup, tce, tdice, ps_loss, l_unc), ce_k)   # :295-306
             self.grads.zero()                                                                    # :285
             loss.backward()                                                                      # :287
         self.packer.finalize(x_l.device)                     # (first iteration only: the recorded requests -> device job table)
@@ -421,6 +445,8 @@ class UAPSTrainer:
             cw1, cw2 = self.consistency_weights()                                                # :279-280
             loss_u, ps_loss, l_unc, _, _ = uaps_unlabeled_loss(out_u, mix_w, cw1, cw2, group=self.group)  # :223-277
             loss = sup + loss_u                                                                  # :282
+            if self.log_state is not None:
+                self._log_iteration(out_l[0], y_l, (loss, sup, tce, tdice, ps_loss, l_unc), ce_k)   # :295-306
             self.grads.zero()                                                                    # :285
             loss.backward()                                                                      # :287
         self._reduce_gradients()
@@ -439,3 +465,50 @@ class UAPSTrainer:
     def skipped_steps(self) -> int:
         """How many optimizer updates the device-side guard has skipped so far (synchronises)."""
         return 0 if self.state is None else int(self.state.read().n_skipped)
+
+    # ---- training log (UAPS_train.py:295-364): per-iteration rows on the device, one read-out per epoch ---------------
+    def _log_iteration(self, logits, y_l, scalars, ce_k) -> None:
+        """Device work only: the validation head appends the labeled batch's confusion counts of the main output as row
+        r = log_state[0] of ``log_counts``; ``uaps_val_scalars`` then copies the iteration's scalars to row r of
+        ``log_scalars``."""
+        append_row(logits.detach(), y_l, self.log_counts, self.log_state, self._log_ws)
+        src, table = [*(t.detach() for t in scalars), *ce_k.detach().unbind()], self.log_scalars
+        if len(src) != table.shape[1]:
+            raise RuntimeError(f"the training log has {table.shape[1]} scalar columns, the iteration gave {len(src)}")
+        with L.on_device(logits.device):
+            L.check(L.lib().uaps_val_scalars(L.ptr_array(src), len(src), table.data_ptr(), table.shape[0],
+                                             self.log_state.data_ptr(), L.stream_ptr()), "uaps_val_scalars")
+
+    def _require_log(self) -> None:
+        if self.log_state is None:
+            raise RuntimeError("the training log is off: construct the trainer with UAPSConfig(train_log_rows=n), n > 0")
+
+    @torch.no_grad()
+    def log_begin(self) -> None:
+        """Start an epoch of the training log: clears its tables (in place: a captured iteration keeps writing to them)."""
+        self._require_log()
+        self.log_counts.zero_()
+        self.log_scalars.zero_()
+        self.log_state.zero_()
+
+    def log_result(self) -> Dict[str, object]:
+        """The means over the iterations since ``log_begin()`` of what the reference logs per iteration (:295-306) and
+        averages per epoch (:316-327): {"loss", "supervised_loss", "total_loss_ce", "total_loss_dice", "ps_loss",
+        "l_uncert", "loss_ce_k" (K floats), "pixel_accuracy", "mIoU", "mDice", "iterations"}.  The metrics are those of
+        the labeled batch's main-decoder logits, the reference's formulas per iteration, then averaged; under
+        torch.distributed each iteration's counts are summed over the ranks first (the whole global batch, as
+        DataParallel's gather), while the loss scalars are already global-batch values on every rank.  One all-reduce
+        (N > 1) and one host sync.
+
+        These are true means.  The reference runs 59 iterations per epoch but divides its sums by 60 (:159, :316-327);
+        its figure is ``value * iterations / 60``.
+
+        Raises when more iterations ran than ``train_log_rows``, when a label was outside [0, C) and not -100, when the
+        ranks logged different numbers of iterations, or when no iteration was logged."""
+        self._require_log()
+        res = finalize(self.log_counts, self.log_state, self.group, scalars=self.log_scalars, errors=_LOG_ERRORS)
+        s = res["scalars"]
+        out: Dict[str, object] = dict(zip(LOG_SCALARS, s))
+        out["loss_ce_k"] = s[len(LOG_SCALARS):]
+        out.update(pixel_accuracy=res["pixel_accuracy"], mIoU=res["mIoU"], mDice=res["mDice"], iterations=res["batches"])
+        return out

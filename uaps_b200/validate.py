@@ -17,7 +17,7 @@ the counts of the WHOLE batch i -- what DataParallel's gather to GPU 0 gives the
 """
 from __future__ import annotations
 
-from typing import Dict
+from typing import Dict, Optional
 
 import torch
 import torch.distributed as dist
@@ -37,16 +37,29 @@ def _world(group):
     return world, (dist.get_rank(group) if world > 1 else 0)
 
 
-def finalize(table: torch.Tensor, state: torch.Tensor, group=None) -> Dict[str, float]:
+VAL_ERRORS = {"ranks": "the ranks validated different numbers of batches",
+              "overflow": "more validation batches than max_batches since begin()",
+              "empty": "no validation batch since begin()"}
+
+
+def finalize(table: torch.Tensor, state: torch.Tensor, group=None, scalars: Optional[torch.Tensor] = None,
+             errors: Dict[str, str] = VAL_ERRORS) -> Dict[str, float]:
     """The epoch's result from the table ``uaps_val_fold`` fills: fp64 [max_batches, C*C + 3] rows of C*C confusion counts
     | CE sum | non-ignored pixels | pixels, and ``state`` = (rows written, overflow flag, bad labels).  Plain torch ops on
     whatever device the tensors live on; the only host sync is the final read-out.  With a process group of N > 1 ranks
     the table and the state are summed over the ranks in ONE all-reduce first; every rank must have written the same
-    number of rows."""
+    number of rows.
+
+    ``scalars``: an optional [max_batches, S] table row-aligned with ``table`` (``uaps_val_scalars``); the result then also
+    holds ``"scalars"``, its S column means over the written rows, read out in the same sync.  These are this rank's own
+    values and are not summed over the ranks.  ``errors``: the messages raised for mismatched row counts, overflow and an
+    empty table."""
     world, rank = _world(group)
     C = int(round((table.shape[1] - 3) ** 0.5))
     if C * C + 3 != table.shape[1]:
         raise ValueError("table rows must hold C*C + 3 values")
+    if scalars is not None and (scalars.dim() != 2 or scalars.shape[0] != table.shape[0]):
+        raise ValueError("the scalar table must have one row per row of the counts table")
     ext = torch.zeros(world + 2, dtype=torch.float64, device=table.device)
     ext[rank] = state[0]                                      # each rank's row count in its own slot: compared after the sum
     ext[world:] = state[1:3]
@@ -59,19 +72,47 @@ def finalize(table: torch.Tensor, state: torch.Tensor, group=None) -> Dict[str, 
     ce = tab[:, C * C] / tab[:, C * C + 1]                    # 0 / 0 = NaN when every pixel is ignored, as torch
     per_row = torch.stack([ce + (1 - mdice), ce, acc, miou, mdice], 1)
     written = (torch.arange(table.shape[0], device=table.device) < n)[:, None]
-    means = torch.where(written, per_row, torch.zeros((), dtype=torch.float64, device=table.device)).sum(0) / n.clamp(min=1)
+    zero = torch.zeros((), dtype=torch.float64, device=table.device)
+    if scalars is not None:
+        per_row = torch.cat([per_row, scalars.double()], 1)
+    means = torch.where(written, per_row, zero).sum(0) / n.clamp(min=1)
     host = torch.cat([means, ext]).tolist()                   # the one host sync
-    rows, overflow, bad = [int(v) for v in host[5:5 + world]], host[5 + world], host[6 + world]
+    m = means.numel()
+    rows, overflow, bad = [int(v) for v in host[m:m + world]], host[m + world], host[m + world + 1]
     if len(set(rows)) != 1:
-        raise RuntimeError(f"the ranks validated different numbers of batches: {rows}")
+        raise RuntimeError(f"{errors['ranks']}: {rows}")
     if overflow:
-        raise RuntimeError("more validation batches than max_batches since begin()")
+        raise RuntimeError(errors["overflow"])
     if bad:
         raise RuntimeError(f"{int(bad)} labels outside [0, C) that are not the ignore index {IGNORE_INDEX}")
     if rows[0] == 0:
-        raise RuntimeError("no validation batch since begin()")
-    return {"val_loss": host[0], "ce": host[1], "pixel_accuracy": host[2], "mIoU": host[3], "mDice": host[4],
-            "batches": rows[0]}
+        raise RuntimeError(errors["empty"])
+    res = {"val_loss": host[0], "ce": host[1], "pixel_accuracy": host[2], "mIoU": host[3], "mDice": host[4],
+           "batches": rows[0]}
+    if scalars is not None:
+        res["scalars"] = host[5:m]
+    return res
+
+
+def append_row(logits: torch.Tensor, y: torch.Tensor, table: torch.Tensor, state: torch.Tensor,
+               workspaces: Dict[tuple, torch.Tensor]) -> None:
+    """The validation head on one batch: fp32 logits [B, C, H, W] and int64 labels ([B, H, W] or [B, H*W]) become the
+    next row of ``table`` (``uaps_val_counts`` + ``uaps_val_fold``).  ``workspaces``: the caller's cache of head
+    workspaces per (B, H*W); a missing one is allocated here, so call once eagerly per shape before a graph capture."""
+    B, C, H, W = logits.shape
+    if table.shape[1] != C * C + 3:
+        raise ValueError(f"table rows hold {table.shape[1]} values, the logits' {C} classes need {C * C + 3}")
+    logits, y = logits.contiguous(), y.reshape(B, H * W).contiguous()
+    lib = L.lib()
+    ws = workspaces.get((B, H * W))
+    if ws is None:
+        ws = torch.empty(lib.uaps_val_workspace_bytes(C, B, H * W), dtype=torch.uint8, device=logits.device)
+        workspaces[(B, H * W)] = ws
+    with L.on_device(logits.device):
+        L.check(lib.uaps_val_counts(logits.data_ptr(), y.data_ptr(), B, C, H * W, ws.data_ptr(), ws.numel(),
+                                    L.stream_ptr()), "uaps_val_counts")
+        L.check(lib.uaps_val_fold(ws.data_ptr(), ws.numel(), B, C, H * W, table.data_ptr(), table.shape[0],
+                                  state.data_ptr(), L.stream_ptr()), "uaps_val_fold")
 
 
 def _owned_layer(w, b, cin_split=None):
@@ -180,14 +221,4 @@ class Validator:
         return self._graphs[key]
 
     def _head(self, logits: torch.Tensor, y: torch.Tensor) -> None:
-        B, C, H, W = logits.shape
-        lib = L.lib()
-        ws = self._ws.get((B, H * W))
-        if ws is None:
-            ws = torch.empty(lib.uaps_val_workspace_bytes(C, B, H * W), dtype=torch.uint8, device=logits.device)
-            self._ws[(B, H * W)] = ws
-        with L.on_device(logits.device):
-            L.check(lib.uaps_val_counts(logits.data_ptr(), y.data_ptr(), B, C, H * W, ws.data_ptr(), ws.numel(),
-                                        L.stream_ptr()), "uaps_val_counts")
-            L.check(lib.uaps_val_fold(ws.data_ptr(), ws.numel(), B, C, H * W, self.table.data_ptr(), self.max_batches,
-                                      self.state.data_ptr(), L.stream_ptr()), "uaps_val_fold")
+        append_row(logits, y, self.table, self.state, self._ws)
