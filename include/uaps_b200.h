@@ -542,6 +542,40 @@ int uaps_unet_ensemble_run(const void* state, size_t state_bytes, int in_chns, i
 int uaps_unet_ensemble_layer(int in_chns, int C, int n_aux, int layer, size_t* weight_offset, size_t* bias_offset,
                              size_t* packed_offset, size_t* packed_bytes);
 
+/* ---------------------------------------------------------------------------------------------
+ * Defect regions: the connected components of a label map, the step from pixel maps (uaps_ensemble_head,
+ * uaps_unet_infer_run, uaps_unet_ensemble_run) to the defects an inspection line acts on.
+ *   labels [B, H, W] uint8; class 0 is background.  A region is a maximal 8-connected set of pixels that all have the
+ *     same nonzero label (touching pixels of different nonzero classes belong to different regions).
+ *   regions [B, H, W] int32: the region id of each pixel, 0 for background.  Within each image the ids are 1..n in
+ *     raster order of the regions' first pixels (smallest y * W + x), so they do not depend on scheduling: the map,
+ *     count and every integer statistic are bitwise reproducible.
+ *   count [B] int32: n, the true region count of each image, also when it exceeds max_regions.
+ *   stats [B, max_regions] UapsRegion in id order: class, area, the half-open box [y0, y1) x [x0, x1) (as
+ *     scipy.ndimage.find_objects slices) and unc_mean, the mean of `uncertainty` over the region (summed in fp64,
+ *     sum / area rounded once to fp32; 0 when uncertainty is NULL).  Rows count .. max_regions - 1 are zero-filled on
+ *     every call; regions past max_regions keep their ids in the map but get no row.  stats is NULL iff max_regions == 0.
+ *   uncertainty [B, H, W] fp32, nullable (e.g. the uncertainty map of uaps_unet_ensemble_run).
+ * Any H, W >= 1 with H * W < 2^31, B <= 65535.  regions, count, stats, uncertainty 4-byte aligned; workspace: >=
+ * uaps_regions_workspace_bytes(B, H, W, max_regions) bytes, 8-byte aligned.  Neither workspace nor outputs need
+ * initialisation.  Every argument is checked before the first launch and the launch sequence depends on the arguments
+ * only, so the call can be captured into a CUDA graph (after uaps_unet_ensemble_run) and replayed with new labels.
+ * Seven launches or fewer: tile-local union-find in shared memory, unions across tile borders, path flattening, a
+ * per-image scan of the roots, ids, relabel + statistics, means.  uaps_regions_workspace_bytes returns 0 for arguments
+ * outside the supported range.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct UapsRegion {
+    int32_t cls;                 /* the region's class, 1..255                          */
+    int32_t area;                /* pixels                                             */
+    int32_t y0, x0, y1, x1;      /* box, half-open: rows y0 .. y1 - 1, columns x0 .. x1 - 1 */
+    float unc_mean;              /* mean uncertainty over the region (0 without a map)  */
+    int32_t reserved;            /* 0                                                  */
+} UapsRegion;
+size_t uaps_regions_workspace_bytes(int B, int H, int W, int max_regions);
+int uaps_regions(const uint8_t* labels, const float* uncertainty /* nullable */, int B, int H, int W, int32_t* regions,
+                 int32_t* count, UapsRegion* stats /* NULL iff max_regions == 0 */, int max_regions, void* workspace,
+                 size_t workspace_bytes, cudaStream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -112,6 +112,8 @@ _SIGNATURES = {
     "uaps_unet_ensemble_run": (_i, [_vp, C.c_size_t, _i, _i, _i, _vp, _i, _i, _i, _vp, _vp, C.c_size_t, _vp, _vp, _vp, _vp,
                                     _vp]),
     "uaps_unet_ensemble_layer": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "uaps_regions_workspace_bytes": (C.c_size_t, [_i, _i, _i, _i]),
+    "uaps_regions": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _vp, C.c_size_t, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None
